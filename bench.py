@@ -232,6 +232,43 @@ STAT_NAMES = ["cyc_interp", "cyc_me", "cyc_me_bi", "cyc_tx_chain", "cyc_coeff_bi
                                                                                "commit")] + ["me_stage_" + n for n in ("telescope", "candidates", "hexagon", "halfpel", "quarterpel")]
 
 
+DUMP_ARRAY_BYTES = 7_500_000  # per array; eight arrays stay under 64 MB in all
+
+
+def dump_outputs(directory, frames):
+    """--dump-outputs: what tb_rdo_encode_frames returns for the given frames (one GOP), as DIR/<name>.npy for comparing two builds output for
+    output.  Samples become float32, wider integers float64 (both exact).  An array above DUMP_ARRAY_BYTES is replaced by a fixed, seeded sample of
+    its elements (1-D) or rows (2-D): the same positions in every run with the same arguments."""
+    def save(name, a, dtype):
+        a = np.ascontiguousarray(a, dtype=dtype)
+        row = a[0].nbytes if a.ndim > 1 and len(a) else a.itemsize
+        n = max(1, DUMP_ARRAY_BYTES // row)
+        if len(a) > n:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), n, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+    os.makedirs(directory, exist_ok=True)
+    blk_fields = [n for n in frames[0].blk.dtype.names if n != "pad"]
+    leaf_cols = lambda lv: np.concatenate([lv[n].reshape(len(lv), -1).astype(np.float64) for n in lv.dtype.names], axis=1)
+    count = lambda size, split: (4 if split else 1) * min(size // 2 if split else size, 16) ** 2  # coeff_count() of thor_b200/csrc/tb_rdo.h
+    leaves, coeffs = [], []
+    for hf in frames:
+        for s in range(hf.job.nsb):
+            lv = hf.leaves[s, :hf.leaf_count[s]]
+            leaves.append(leaf_cols(lv))
+            for size, split, ofs in zip(lv["size"].astype(int), lv["tb_split"].astype(int), lv["coeff_ofs"].astype(int)):
+                if ofs >= 0:  # a coded block's coefficients: luma, then the two chroma runs; the rest of the area is not written
+                    n = count(size, split) + 2 * count(size // 2, split and size // 2 > 4)
+                    coeffs.append(hf.coeffs[s, ofs:ofs + n])
+    for p, name in enumerate(("rec_y", "rec_u", "rec_v")):
+        save(name, np.concatenate([hf.rec[p].reshape(-1) for hf in frames]), np.float32)
+    save("blk", np.concatenate([np.stack([hf.blk[n].astype(np.float32) for n in blk_fields], axis=1) for hf in frames]), np.float32)
+    save("leaf_count", np.concatenate([hf.leaf_count for hf in frames]), np.float64)
+    save("sb_cost", np.concatenate([[hf.leaves["cost"][s, :hf.leaf_count[s]].astype(np.int64).sum() for s in range(hf.job.nsb)] for hf in frames]), np.float64)
+    save("leaves", np.concatenate(leaves), np.float64)
+    save("coeffs", np.concatenate(coeffs) if coeffs else np.zeros(0, np.int16), np.float32)
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------------------------------
@@ -316,6 +353,12 @@ def run_gpu(args, cfg):
     ck(L.tb_rdo_batch_sync(batch), "timed launch")
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:  # the decisions of the last timed step (its GOP replica), downloaded after the timed region
+        download_last = range(nfr * (K - 1), nfr * K)
+        for s in download_last:
+            ck(L.tb_rdo_batch_download(batch, s, C.byref(hosts[s].desc)), "tb_rdo_batch_download")
+        ck(L.tb_rdo_batch_sync(batch), "download of the last step")
+        dump_outputs(args.dump_outputs, [hosts[s] for s in download_last])
     stats = (C.c_uint64 * len(STAT_NAMES))()
     L.tb_rdo_batch_stats(batch, stats, len(STAT_NAMES))
     st = dict(zip(STAT_NAMES, [int(v) for v in stats]))
@@ -621,7 +664,12 @@ def main():
     ap.add_argument("--cache", default=os.environ.get("THOR_B200_CACHE", "/tmp/thor_b200_bench"))
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-fresh", action="store_true", help="cpu_baseline: measure again even if a recent measurement of this box exists in the cache")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the decisions of the last timed step (reconstruction, block state, leaves, coefficients, RD costs) "
+                         "as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = Cfg(args.config, tuple(int(v) for v in args.size.split("x")) if args.size else None, args.frames or None)
     os.makedirs(args.cache, exist_ok=True)
     if args.impl == "reference":
