@@ -32,12 +32,12 @@ def _compile(src, obj, flags):
     return r.returncode, " ".join(cmd) + "\n" + r.stdout + r.stderr
 
 
-def build(force=False, verbose=False, defines=(), out=None):
+def build(force=False, verbose=False, out=None):
     """one object per translation unit (compiled in parallel, kept under thor_b200/build/ and reused while its sources are older), then one link"""
     if not force and not stale() and out is None:
         return LIB
     from concurrent.futures import ThreadPoolExecutor
-    flags = [f for f in NVCC_FLAGS if not f.startswith("--use_fast_math") and f != "-shared"] + ["-D" + d for d in defines]
+    flags = [f for f in NVCC_FLAGS if not f.startswith("--use_fast_math") and f != "-shared"]
     objdir = os.path.join(HERE, "build", "default" if out is None else os.path.basename(out))
     os.makedirs(objdir, exist_ok=True)
     newest = max(os.path.getmtime(os.path.join(CSRC, d)) for d in DEPS)

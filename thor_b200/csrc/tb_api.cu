@@ -401,11 +401,11 @@ int tb_motion_estimate_batch(const tb_me_item_t *items, int n, const int16_t *ca
   idx = meta + 128;
   CKB(cudaMemsetAsync(meta, 0, 128 * sizeof(int), g.stream), "me scratch");
   const int sgrid = std::min((n + 255) / 256, g.sm_count * 8);
-  const MeClassOf cls{speed, (TB_ME_QUAD && sample_bytes == 1 && speed == 0) ? 1 : 0};
+  const MeClassOf cls{speed, (sample_bytes == 1 && speed == 0) ? 1 : 0};
   LAUNCH((sched_hist_kernel<tb_me_item_t, MeClassOf>), sgrid, 256, 0, items, n, cls, meta);
   LAUNCH(sched_scan_kernel, 1, 32, 0, meta);
   LAUNCH((sched_scatter_kernel<tb_me_item_t, MeClassOf>), sgrid, 256, 0, items, n, cls, meta, idx);
-  const int grid = std::min((n + WARPS_PER_CTA - 1) / WARPS_PER_CTA, g.sm_count * TB_ME_MINBLOCKS);  // persistent: every CTA resident
+  const int grid = std::min((n + WARPS_PER_CTA - 1) / WARPS_PER_CTA, g.sm_count * ME_MINBLOCKS);  // persistent: every CTA resident
   if (sample_bytes == 1) LAUNCH(me_batch_kernel<uint8_t>, grid, CTA_THREADS, 0, items, n, idx, meta, cand, bitdepth, speed, bip, fw, fh, out, g.me_stats);
   else LAUNCH(me_batch_kernel<uint16_t>, grid, CTA_THREADS, 0, items, n, idx, meta, cand, bitdepth, speed, bip, fw, fh, out, g.me_stats);
   CKB(cudaFreeAsync(meta, g.stream), "me scratch");
@@ -453,7 +453,7 @@ int tb_txfm_chain_batch(const tb_txfm_item_t *items, int n, int sample_bytes, in
   LAUNCH((sched_hist_kernel<tb_txfm_item_t, TxClassOf>), sgrid, 256, 0, items, n, cls, meta);
   LAUNCH(sched_scan_kernel, 1, 32, 0, meta);
   LAUNCH((sched_scatter_kernel<tb_txfm_item_t, TxClassOf>), sgrid, 256, 0, items, n, cls, meta, idx);
-  const int grid = std::min((n + 31) / 32, g.sm_count * TB_TX_MINBLOCKS);  // persistent: every CTA resident
+  const int grid = std::min((n + 31) / 32, g.sm_count * TX_MINBLOCKS);  // persistent: every CTA resident
   if (sample_bytes == 1) LAUNCH(txfm_chain_kernel<uint8_t>, grid, CTA_THREADS, smem, items, n, idx, meta, bitdepth, out);
   else LAUNCH(txfm_chain_kernel<uint16_t>, grid, CTA_THREADS, smem, items, n, idx, meta, bitdepth, out);
   CKB(cudaFreeAsync(meta, g.stream), "txfm scratch");

@@ -12,39 +12,6 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
-#ifndef TB_EXP_NOSUBPEL
-#define TB_EXP_NOSUBPEL 0  // 1: skip the sub-pel SADs (timing experiment only: measures the integer stages alone)
-#endif
-#ifndef TB_ME_QUAD
-#define TB_ME_QUAD 1  // four searches per warp for 8-bit blocks of <= 64 samples (quad_motion_estimate)
-#endif
-#ifndef TB_ME_QUAD_SIZE16
-#define TB_ME_QUAD_SIZE16 1  // also the 8x8 partitions of 16x16 coding blocks (wide-SAD candidate stage)
-#endif
-#ifndef TB_QUAD_HALFPEL_PLANES
-#define TB_QUAD_HALFPEL_PLANES 0  // group form of the half-pel planes inside quad_motion_estimate: bit-exact, measured slower (cb8 class 6.2 vs 5.3 ms)
-#endif
-#ifndef TB_SAD_V4
-#define TB_SAD_V4 1  // 128-bit loads for block rows of >= 16 bytes
-#endif
-#ifndef TB_HALFPEL_PLANES
-#define TB_HALFPEL_PLANES 1  // half-pel stage from three shared planes (halfpel_stage_sads_u8)
-#endif
-#ifndef TB_SUBPEL_SHARED
-// 1: sub-pel stages through subpel_stage_sads_shared (horizontally filtered rows shared between the eight probes via shared
-// memory).  Bit-exact, but measured SLOWER on B200 (sub-pel share of the 1080p batch 9.4 ms vs 6.8 ms): per 16x16 tile it
-// executes only ~1.2x fewer instructions than the per-probe register form (22 filtered rows per 16 output rows, five planes)
-// and adds two shared-memory round trips per tile to every warp's dependency chain; 22 KB of shared memory per CTA also
-// shrinks L1.  Kept as a measured alternative.
-#define TB_SUBPEL_SHARED 0
-#endif
-#ifndef TB_TX_MINBLOCKS
-#define TB_TX_MINBLOCKS 6  // __launch_bounds__(128, N) of the transform-chain kernel (measured: 4: 5.84 ms, 5: 5.37, 6: 5.12)
-#endif
-#ifndef TB_ME_MINBLOCKS
-#define TB_ME_MINBLOCKS 6  // __launch_bounds__(128, N) of the motion-search kernel: registers/thread <= 65536 / (128 N)
-#endif
-
 // TB_LDG: read-only-path load of data that no thread writes during the kernel (frames, work items).  TB_LDF: load of reconstructed
 // samples that ANOTHER CTA may have written earlier in the same kernel (wavefront RD loop, tb_rdo.cu): that translation unit maps
 // TB_LDG to a plain load (its "original" block can be a scratch block written moments ago) and TB_LDF to an L1-bypassing load.
@@ -146,7 +113,6 @@ __device__ __forceinline__ uint32_t sad_partial(const S *o, int os, const S *r, 
   const uint32_t *rq = (const uint32_t *)(ra & ~(uintptr_t)3);
   const uint32_t *oq = (const uint32_t *)o;
   const int rsw = (rs * (int)sizeof(S)) >> 2, osw = (os * (int)sizeof(S)) >> 2;  // pitches in words
-#if TB_SAD_V4
   if (V4 && !(ww & 3) && !((((uintptr_t)o) | (unsigned)(osw << 2) | (unsigned)(rsw << 2)) & 15)) {
     const uint4 *rv = (const uint4 *)(ra & ~(uintptr_t)15), *ov = (const uint4 *)o;
     const unsigned sh8 = (unsigned)(ra & 3) * 8;
@@ -157,7 +123,6 @@ __device__ __forceinline__ uint32_t sad_partial(const S *o, int os, const S *r, 
       default: return sad_rows_v4<S, 3>(rv, rsw >> 2, ov, osw >> 2, ww >> 2, h, sub, nl, sh8);
     }
   }
-#endif
   uint32_t acc = 0;
   TB_ROLL
   for (int row = sub; row < h; row += nl) {
@@ -291,11 +256,9 @@ __device__ __noinline__ uint32_t multi_sad_rows(const S *o, int os, const S *r, 
 }
 template <class S, int TW = 1>
 __device__ __forceinline__ uint32_t multi_sad(const S *o, int os, const S *r, int rs, int w, int h, int roff, int n) {
-#if TB_SAD_V4
   // only the CTA-team searches (blocks >= 2048 samples) take the wide form: a second callee at the call sites of the one-warp
   // searches costs them more in spills than the 32x32 blocks would gain
   if (TW > 1 && (w / Word<S>::PW) * h >= 256 && h >= 16 && w * (int)sizeof(S) >= 16) return multi_sad_wide<S>(o, os, r, rs, w, h, roff, n);
-#endif
 #if TB_SAD_ROWS
   if (TW == 1 && w / Word<S>::PW >= 8) return multi_sad_rows<S>(o, os, r, rs, w, h, roff, n);
 #endif
@@ -579,163 +542,6 @@ __device__ __noinline__ uint32_t subpel_stage_sads(const S *o, int os, const S *
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// One whole sub-pel stage (the eight probes around a centre, enc/encode_block.c:625-663) for 8-bit samples with the
-// horizontally filtered rows SHARED between probes.  The eight probes use at most three distinct horizontal filters
-// (x offsets -d, 0, +d), and the (2,2) positions use the two row filters of the 12-tap centre kernel, so per 16 x 16
-// tile of the block the warp
-//   (H) filters each needed row ONCE per distinct (filter, integer column) into int16 planes in shared memory
-//       (<= 7 planes of (16 + 6) rows; one (plane, row, 4-sample strip) unit per lane and step), then
-//   (V) runs the vertical 6-tap pass of every probe from those planes: four lanes (or more, when fewer probes take a
-//       pass) per probe, one (row, strip) unit per lane and step, DP2A on the int16 pairs, I2IP pack, VABSDIFF4 against
-//       the original word.
-// A horizontally filtered row is computed 3 (+2) times per stage instead of 8, and small blocks keep all lanes busy
-// (a 4x4 block is 50 + 32 units instead of eight serial 9-row strips).  Lane t < 8 returns the SAD of probe t + 1.
-// ---------------------------------------------------------------------------------------------------------------
-struct alignas(16) SubpelShared {
-  int16_t plane[7][22][16];  // [slot][row][column]; row 0 = reference row (first block row + vmin - 2)
-  uint32_t pd[8][8];         // probe t: K0..K5 (vertical taps as DP2A words), slot | rowoff << 8, unused
-  uint32_t gd[6][4];         // H group: integer column offset, taps lo, taps hi, slot | pair << 8
-  uint32_t sad[8];
-  uint8_t list[2][8];        // probes of the standard / centre-kernel pass
-};
-constexpr int SUBPEL_TR = 16, SUBPEL_TW = 16;
-
-__device__ __noinline__ uint32_t subpel_stage_sads_shared(const uint8_t *o, int os, const uint8_t *ref, int rs, int w, int hfull, int cx0, int cy0, const int8_t *dxs,
-                                                          const int8_t *dys, int sign, int bip, int pic_w, int pic_h, int xpos, int ypos, int row0, int h, SubpelShared &sh) {
-  const int lane = lane_id(), t = lane & 7;
-  // ---- probe geometry (lanes 0..7; lanes 8..15 carry the centre-kernel requests of the same probes)
-  const int mvx = (int)(int16_t)(cx0 + dxs[t + 1]), mvy = (int)(int16_t)(cy0 + dys[t + 1]);
-  int hi, vi, xf, yf;
-  split_mv(mvx, mvy, sign, 2, pic_w, pic_h, xpos, ypos, w, hfull, hi, vi, xf, yf);
-  const bool special = xf == 2 && yf == 2 && bip < 2;
-  const int vmin = __reduce_min_sync(FULL, vi), vmax = __reduce_max_sync(FULL, vi), himin = __reduce_min_sync(FULL, hi);
-  const bool is_std_req = lane < 8 && !special, is_pair_req = lane >= 8 && lane < 16 && special;
-  const uint32_t key = is_std_req ? (uint32_t)(xf << 20) + (uint32_t)(hi - himin) : (is_pair_req ? 0x40000000u + (uint32_t)(hi - himin) : 0x7f000000u + lane);
-  const unsigned same = __match_any_sync(FULL, key);
-  const int leader_lane = __ffs(same) - 1;
-  const bool leader = leader_lane == lane;
-  const unsigned std_leaders = __ballot_sync(FULL, leader && is_std_req), pair_leaders = __ballot_sync(FULL, leader && is_pair_req);
-  const unsigned lt = (1u << lane) - 1;
-  const int nstd = __popc(std_leaders), npair = __popc(pair_leaders), G = nstd + npair;
-  int slot = is_std_req ? __popc(std_leaders & lt) : nstd + 2 * __popc(pair_leaders & lt);
-  const int grp = is_std_req ? __popc(std_leaders & lt) : nstd + __popc(pair_leaders & lt);
-  slot = __shfl_sync(FULL, slot, leader_lane);
-  const int pair_slot = __shfl_sync(FULL, slot, 8 + t);
-  if (vmax - vmin > 1 || nstd + 2 * npair > 7 || (h & 3) || (w & 3)) return 0xffffffffu;  // caller falls back to the per-probe form
-  if (leader && (is_std_req || is_pair_req)) {
-    const int8_t *fh = c_luma_taps[bip ? 1 : 0][xf];
-    sh.gd[grp][0] = (uint32_t)hi;
-    sh.gd[grp][1] = is_std_req ? pack_s8x4(fh[0], fh[1], fh[2], fh[3]) : 0;
-    sh.gd[grp][2] = is_std_req ? pack_s8x4(fh[4], fh[5], 0, 0) : 0;
-    sh.gd[grp][3] = (uint32_t)slot | (is_pair_req ? 0x100u : 0u);
-  }
-  const unsigned std_probes = __ballot_sync(FULL, lane < 8 && !special), spec_probes = __ballot_sync(FULL, lane < 8 && special);
-  if (lane < 8) {
-    const int8_t *fv = c_luma_taps[bip ? 1 : 0][yf];
-#pragma unroll
-    for (int m = 0; m < 6; m++) sh.pd[lane][m] = (uint32_t)(fv[m] & 0xff) | ((uint32_t)(fv[m] & 0xff) << 24);
-    sh.pd[lane][6] = (uint32_t)(special ? pair_slot : slot) | ((uint32_t)(vi - vmin) << 8);
-    if (special) sh.list[1][__popc(spec_probes & lt)] = (uint8_t)lane;
-    else sh.list[0][__popc(std_probes & lt)] = (uint8_t)lane;
-  }
-  __syncwarp();
-  const int nsp = __popc(std_probes), nxp = __popc(spec_probes);
-  // lanes per probe in each pass: the largest power of two with (probes x lanes) <= 32
-  const int lp_s = nsp ? 1 << ilog2(32 / nsp) : 32, lp_x = nxp ? 1 << ilog2(32 / nxp) : 32;
-  const int ks = lane / lp_s, subs = lane & (lp_s - 1), kx = lane / lp_x, subx = lane & (lp_x - 1);
-  const bool act_s = ks < nsp, act_x = kx < nxp;
-  uint32_t K[6], meta_s = 0, meta_x = 0;
-  if (act_s) {
-    const int ps = sh.list[0][ks];
-#pragma unroll
-    for (int m = 0; m < 6; m++) K[m] = sh.pd[ps][m];
-    meta_s = sh.pd[ps][6];
-  }
-  if (act_x) meta_x = sh.pd[sh.list[1][kx]][6];
-  uint32_t acc_s = 0, acc_x = 0;
-  const uint8_t *rbase = ref + (row0 + vmin - 2) * rs;  // plane row 0 of the first tile
-  for (int ty = 0; ty < h; ty += SUBPEL_TR) {
-    const int tr = min(SUBPEL_TR, h - ty), R = tr + 6;
-    for (int tx = 0; tx < w; tx += SUBPEL_TW) {
-      const int ns = min(SUBPEL_TW, w - tx) >> 2, lns = ilog2(ns), RN = R * ns, inv = 65536 / RN + 1, total = G * RN;
-      // ---- (H)
-      for (int u = lane; u < total; u += 32) {
-        const int g = (u * inv) >> 16, rem = u - g * RN, r = rem >> lns, st = rem & (ns - 1);
-        const uint4 gd = *(const uint4 *)sh.gd[g];
-        const uint8_t *p = rbase + (ty + r) * rs + (int)gd.x + tx + 4 * st;
-        const int sl = gd.w & 0xff;
-        uintptr_t a = (uintptr_t)(p - 2);
-        const uint32_t *wq = (const uint32_t *)(a & ~(uintptr_t)3);
-        const unsigned shb = (unsigned)(a & 3) * 8;
-        const uint32_t w0 = TB_LDG(wq), w1 = TB_LDG(wq + 1), w2 = TB_LDG(wq + 2), w3 = TB_LDG(wq + 3);
-        const uint32_t b0 = __funnelshift_r(w0, w1, shb), b1 = __funnelshift_r(w1, w2, shb), b2 = __funnelshift_r(w2, w3, shb);
-        if (gd.w & 0x100) {  // the two row filters of the centre kernel: H1 = [0 0 1 1 0 0], H2 = [0 1 2 2 1 0]
-          const uint32_t a_lo = 0x01010000u, b_lo = 0x02020100u, b_hi = 0x00000001u;
-          int h1[4], h2[4];
-#pragma unroll
-          for (int k = 0; k < 4; k++) {
-            uint32_t lo = __funnelshift_r(b0, b1, 8 * k), hi4 = __funnelshift_r(b1, b2, 8 * k);
-            h1[k] = dp4a_us(lo, a_lo, 0);
-            h2[k] = dp4a_us(lo, b_lo, dp4a_us(hi4, b_hi, 0));
-          }
-          *(uint2 *)&sh.plane[sl][r][4 * st] = make_uint2((uint32_t)h1[0] | ((uint32_t)h1[1] << 16), (uint32_t)h1[2] | ((uint32_t)h1[3] << 16));
-          *(uint2 *)&sh.plane[sl + 1][r][4 * st] = make_uint2((uint32_t)h2[0] | ((uint32_t)h2[1] << 16), (uint32_t)h2[2] | ((uint32_t)h2[3] << 16));
-        } else {
-          int hv[4];
-#pragma unroll
-          for (int k = 0; k < 4; k++) {
-            uint32_t lo = __funnelshift_r(b0, b1, 8 * k), hi4 = __funnelshift_r(b1, b2, 8 * k);
-            hv[k] = dp4a_us(lo, gd.y, dp4a_us(hi4, gd.z, 0));
-          }
-          *(uint2 *)&sh.plane[sl][r][4 * st] = make_uint2(((uint32_t)hv[0] & 0xffffu) | ((uint32_t)hv[1] << 16), ((uint32_t)hv[2] & 0xffffu) | ((uint32_t)hv[3] << 16));
-        }
-      }
-      __syncwarp();
-      // ---- (V) standard probes: out = sat((sum_m fv[m] * H[y - 2 + m] + 2048) >> 12)
-      if (act_s) {
-        const int sl = meta_s & 0xff, ro = (meta_s >> 8) & 0xff;
-        for (int u = subs; u < tr * ns; u += lp_s) {
-          const int y = u >> lns, st = u & (ns - 1);
-          int a0 = 2048, a1 = 2048, a2 = 2048, a3 = 2048;
-#pragma unroll
-          for (int m = 0; m < 6; m++) {
-            const uint2 hw = *(const uint2 *)&sh.plane[sl][ro + y + m][4 * st];
-            a0 = __dp2a_lo((int)hw.x, (int)K[m], a0);
-            a1 = __dp2a_hi((int)hw.x, (int)K[m], a1);
-            a2 = __dp2a_lo((int)hw.y, (int)K[m], a2);
-            a3 = __dp2a_hi((int)hw.y, (int)K[m], a3);
-          }
-          const uint32_t pk = pack_sat_u8x4(a0 >> 12, a1 >> 12, a2 >> 12, a3 >> 12);
-          acc_s += __vsadu4(TB_LDG((const uint32_t *)(o + (row0 + ty + y) * os + tx + 4 * st)), pk);
-        }
-      }
-      // ---- (V) centre-kernel probes: out = (H1[y-1] + H2[y] + H2[y+1] + H1[y+2] + 8) >> 4   (<= 255: no clamp needed)
-      if (act_x) {
-        const int sl = meta_x & 0xff, ro = (meta_x >> 8) & 0xff;
-        for (int u = subx; u < tr * ns; u += lp_x) {
-          const int y = u >> lns, st = u & (ns - 1);
-          const uint2 p0 = *(const uint2 *)&sh.plane[sl][ro + y + 1][4 * st], p3 = *(const uint2 *)&sh.plane[sl][ro + y + 4][4 * st];
-          const uint2 p1 = *(const uint2 *)&sh.plane[sl + 1][ro + y + 2][4 * st], p2 = *(const uint2 *)&sh.plane[sl + 1][ro + y + 3][4 * st];
-          const uint32_t s01 = ((p0.x + p1.x + p2.x + p3.x + 0x00080008u) >> 4) & 0x0fff0fffu;  // packed u16 pairs, sums <= 4088
-          const uint32_t s23 = ((p0.y + p1.y + p2.y + p3.y + 0x00080008u) >> 4) & 0x0fff0fffu;
-          const uint32_t pk = __byte_perm(s01, s23, 0x6420);
-          acc_x += __vsadu4(TB_LDG((const uint32_t *)(o + (row0 + ty + y) * os + tx + 4 * st)), pk);
-        }
-      }
-      __syncwarp();
-    }
-  }
-  acc_s = group_sum(acc_s, lp_s);
-  acc_x = group_sum(acc_x, lp_x);
-  if (act_s && subs == 0) sh.sad[sh.list[0][ks]] = acc_s;
-  if (act_x && subx == 0) sh.sad[sh.list[1][kx]] = acc_x;
-  __syncwarp();
-  const uint32_t out = sh.sad[t];
-  __syncwarp();
-  return out;
-}
-
-// ---------------------------------------------------------------------------------------------------------------
 // The half-pel stage (enc/encode_block.c:625-645) for 8-bit samples when the centre is an integer position: its eight
 // probes read only THREE interpolated planes — the horizontal half-pel plane (probes (0,-2), (0,+2) in (dy,dx)), the vertical
 // one ((-2,0), (+2,0)) and the 12-tap centre-kernel plane (the four diagonals) — each shifted by 0 or 1 sample.  So every plane
@@ -753,22 +559,19 @@ __device__ __forceinline__ void row12_u8(const uint8_t *p, uint32_t &b0, uint32_
   const uint32_t w0 = TB_LDG(w), w1 = TB_LDG(w + 1), w2 = TB_LDG(w + 2), w3 = TB_LDG(w + 3);
   b0 = __funnelshift_r(w0, w1, sh); b1 = __funnelshift_r(w1, w2, sh); b2 = __funnelshift_r(w2, w3, sh);
 }
-// NL = 32: the warp works on one search; NL = 8: each group of eight lanes on its own search (quad_motion_estimate)
-template <int NL>
 __device__ __noinline__ uint32_t halfpel_stage_sads_u8(const uint8_t *o, int os, const uint8_t *ref, int rs, int w, int hfull, int bx, int by, const int8_t *dxs,
                                                        const int8_t *dys, int sign, int bip, int pic_w, int pic_h, int xpos, int ypos, int row0, int h) {
-  const int lane = lane_id(), t = lane & 7, sub = lane & (NL - 1);
-  const unsigned gm = NL == 32 ? FULL : 0xffu << (lane & 24);
+  const int lane = lane_id(), t = lane & 7;
   const int mvx = (int)(int16_t)(bx + dxs[t + 1]), mvy = (int)(int16_t)(by + dys[t + 1]);
   int hi, vi, xf, yf;
   split_mv(mvx, mvy, sign, 2, pic_w, pic_h, xpos, ypos, w, hfull, hi, vi, xf, yf);
-  const int hmin = __reduce_min_sync(gm, hi), vmin = __reduce_min_sync(gm, vi);
+  const int hmin = __reduce_min_sync(FULL, hi), vmin = __reduce_min_sync(FULL, vi);
   const int ho = hi - hmin, vo = vi - vmin;
   const int cls = (xf == 2 && yf == 0) ? 0 : ((xf == 0 && yf == 2) ? 1 : ((xf == 2 && yf == 2) ? 2 : 3));
-  const unsigned mH = __ballot_sync(gm, cls == 0), mV = __ballot_sync(gm, cls == 1);
-  const int voH = __shfl_sync(gm, vo, mH ? __ffs(mH) - 1 : (lane & ~(NL - 1))), hoV = __shfl_sync(gm, ho, mV ? __ffs(mV) - 1 : (lane & ~(NL - 1)));
+  const unsigned mH = __ballot_sync(FULL, cls == 0), mV = __ballot_sync(FULL, cls == 1);
+  const int voH = __shfl_sync(FULL, vo, mH ? __ffs(mH) - 1 : 0), hoV = __shfl_sync(FULL, ho, mV ? __ffs(mV) - 1 : 0);
   const bool ok = bip < 2 && cls != 3 && ho <= 1 && vo <= 1 && (cls != 0 || vo == voH) && (cls != 1 || ho == hoV);
-  if (!__all_sync(gm, ok)) return 0xffffffffu;
+  if (!__all_sync(FULL, ok)) return 0xffffffffu;
   const int8_t *fh = c_luma_taps[bip ? 1 : 0][2];
   const uint32_t tlo = pack_s8x4(fh[0], fh[1], fh[2], fh[3]), thi = pack_s8x4(fh[4], fh[5], 0, 0);
   const int ns = w >> 2, lns = ilog2(ns);
@@ -777,7 +580,7 @@ __device__ __noinline__ uint32_t halfpel_stage_sads_u8(const uint8_t *o, int os,
   uint32_t aH0 = 0, aH1 = 0, aV0 = 0, aV1 = 0, aC00 = 0, aC01 = 0, aC10 = 0, aC11 = 0;  // aC<vo><ho>
   // ---- H pass: block rows y (plane rows y + voH), plane columns 4 s .. 4 s + 4
   if (mH) {
-    for (int u = sub; u < h * ns; u += NL) {
+    for (int u = lane; u < h * ns; u += 32) {
       const int y = u >> lns, st = u & (ns - 1);
       uint32_t b0, b1, b2;
       row12_u8(rb + (y + voH) * rs + 4 * st - 2, b0, b1, b2);
@@ -794,7 +597,7 @@ __device__ __noinline__ uint32_t halfpel_stage_sads_u8(const uint8_t *o, int os,
   }
   // ---- V pass: plane rows r = 0 .. h, plane columns 4 s + hoV .. + 3; row r serves block row r (vo 0) and r - 1 (vo 1)
   if (mV) {
-    for (int u = sub; u < (h + 1) * ns; u += NL) {
+    for (int u = lane; u < (h + 1) * ns; u += 32) {
       const int r = u >> lns, st = u & (ns - 1);
       const uint8_t *p = rb + (r - 2) * rs + 4 * st + hoV;
       const uintptr_t a = (uintptr_t)p;
@@ -819,7 +622,7 @@ __device__ __noinline__ uint32_t halfpel_stage_sads_u8(const uint8_t *o, int os,
   // ---- C pass: plane rows r = 0 .. h, plane columns 4 s .. 4 s + 4
   {
     const uint32_t a_lo = 0x01010000u, b_lo = 0x02020100u, b_hi = 0x00000001u;
-    for (int u = sub; u < (h + 1) * ns; u += NL) {
+    for (int u = lane; u < (h + 1) * ns; u += 32) {
       const int r = u >> lns, st = u & (ns - 1);
       const uint8_t *p = rb + r * rs + 4 * st - 2;
       int acc[5] = {8, 8, 8, 8, 8};
@@ -852,8 +655,8 @@ __device__ __noinline__ uint32_t halfpel_stage_sads_u8(const uint8_t *o, int os,
       }
     }
   }
-  aH0 = __reduce_add_sync(gm, aH0); aH1 = __reduce_add_sync(gm, aH1); aV0 = __reduce_add_sync(gm, aV0); aV1 = __reduce_add_sync(gm, aV1);
-  aC00 = __reduce_add_sync(gm, aC00); aC01 = __reduce_add_sync(gm, aC01); aC10 = __reduce_add_sync(gm, aC10); aC11 = __reduce_add_sync(gm, aC11);
+  aH0 = __reduce_add_sync(FULL, aH0); aH1 = __reduce_add_sync(FULL, aH1); aV0 = __reduce_add_sync(FULL, aV0); aV1 = __reduce_add_sync(FULL, aV1);
+  aC00 = __reduce_add_sync(FULL, aC00); aC01 = __reduce_add_sync(FULL, aC01); aC10 = __reduce_add_sync(FULL, aC10); aC11 = __reduce_add_sync(FULL, aC11);
   if (cls == 0) return ho ? aH1 : aH0;
   if (cls == 1) return vo ? aV1 : aV0;
   return vo ? (ho ? aC11 : aC10) : (ho ? aC01 : aC00);
@@ -972,7 +775,6 @@ struct MeCtx {
   double lambda;
   // work counters for the roofline (not part of the result): integer-position block SADs and sub-pel probes
   unsigned n_int, n_sub;
-  SubpelShared *sps;  // per-warp scratch of the shared-row sub-pel stage (8-bit samples)
 #if TB_ME_STAGE_PROF
   long long cyc[5];   // cycles in telescope / candidates / hexagon / half-pel / quarter-pel (diagnostics of the RD loop)
 #endif
@@ -1154,26 +956,17 @@ __device__ void warp_motion_estimate(const S *orig_full, int os, const S *ref_fu
       const int8_t *dm = stage ? qm : hm, *dn = stage ? qn : hn;
       const int bx = optx, by = opty;
       uint32_t sad = 0xffffffffu;
-#if !TB_EXP_NOSUBPEL && TB_HALFPEL_PLANES
       if (sizeof(S) == 1 && stage == 0 && !((bx | by) & 3))
-        sad = halfpel_stage_sads_u8<32>((const uint8_t *)orig_full, os, (const uint8_t *)ref_full, rs, c.width, c.height, bx, by, dn, dm, c.sign, c.bip, c.fw, c.fh, c.xpos, c.ypos,
+        sad = halfpel_stage_sads_u8((const uint8_t *)orig_full, os, (const uint8_t *)ref_full, rs, c.width, c.height, bx, by, dn, dm, c.sign, c.bip, c.fw, c.fh, c.xpos, c.ypos,
                                     row0, band_h);
-#endif
-#if !TB_EXP_NOSUBPEL && TB_SUBPEL_SHARED
-      if (sad == 0xffffffffu && sizeof(S) == 1 && c.sps)
-        sad = subpel_stage_sads_shared((const uint8_t *)orig_full, os, (const uint8_t *)ref_full, rs, c.width, c.height, bx, by, dn, dm, c.sign, c.bip, c.fw, c.fh, c.xpos,
-                                       c.ypos, row0, band_h, *c.sps);
-#endif
       const int i1 = (lane & 7) + 1;
       const int cy = (int)(int16_t)(by + dm[i1]), cx = (int)(int16_t)(bx + dn[i1]);
-#if !TB_EXP_NOSUBPEL
-      if (sad == 0xffffffffu) {  // 16-bit samples, or a geometry the shared form does not take: one probe per 4-lane group
+      if (sad == 0xffffffffu) {  // 16-bit samples, the quarter-pel stage, or a geometry halfpel_stage_sads_u8 does not take: one probe per 4-lane group
         const int tq = (lane >> 2) + 1;
         const int qy = (int)(int16_t)(by + dm[tq]), qx = (int)(int16_t)(bx + dn[tq]);
         sad = subpel_stage_sads<S>(orig_full, os, ref_full, rs, c.width, c.height, qx, qy, c.sign, c.bip, c.fw, c.fh, c.xpos, c.ypos, c.bitdepth, row0, band_h);
         sad = __shfl_sync(FULL, sad, (lane & 7) * 4);
       }
-#endif
       sad = tm.sum(sad);
       const uint32_t cost = (sad >> shift) + mv_cost(c.lambda, quote_mv_bits(cy - c.mvpy, cx - c.mvpx));
       int yd = 0, xd = 0;
@@ -1350,17 +1143,10 @@ __device__ __noinline__ void quad_motion_estimate(const QuadItem &q, int fw, int
     split_mv(cx, cy, q.sign, 2, fw, fh, q.xpos, q.ypos, q.w, q.h, hi, vi, xf, yf);
     const uint8_t *ip = q.ref + vi * q.rs + hi;
     const int RH = q.h >= 8 ? 8 : q.h, nseg = q.h / RH, units = (q.w >> 2) * nseg;
-    uint32_t sad = 0xffffffffu;
-#if TB_HALFPEL_PLANES && TB_QUAD_HALFPEL_PLANES
-    if (stage == 0 && !((optx | opty) & 3))  // three shared planes instead of eight interpolations; also avoids the centre-kernel / general divergence
-      sad = halfpel_stage_sads_u8<8>(q.orig, q.os, q.ref, q.rs, q.w, q.h, optx, opty, dn, dm, q.sign, bip, fw, fh, q.xpos, q.ypos, 0, q.h);
-#endif
-    if (sad == 0xffffffffu) {
-      sad = 0;
-      for (int u = 0; u < units; u++) {
-        const int strip = u / nseg, seg = u - strip * nseg;
-        sad += strip_sad_subpel_u8(q.orig, q.os, ip, q.rs, strip * 4, seg * RH, RH, xf, yf, bip);
-      }
+    uint32_t sad = 0;
+    for (int u = 0; u < units; u++) {
+      const int strip = u / nseg, seg = u - strip * nseg;
+      sad += strip_sad_subpel_u8(q.orig, q.os, ip, q.rs, strip * 4, seg * RH, RH, xf, yf, bip);
     }
     const uint32_t cost = sad + mv_cost(q.lambda, quote_mv_bits(cy - q.mvpy, cx - q.mvpx));
     int yd = 0, xd = 0;

@@ -9,6 +9,8 @@ namespace tb {
 
 constexpr int WARPS_PER_CTA = 4;
 constexpr int CTA_THREADS = WARPS_PER_CTA * 32;
+constexpr int TX_MINBLOCKS = 6;  // __launch_bounds__(128, N) of the transform-chain kernel (measured: 4: 5.84 ms, 5: 5.37, 6: 5.12)
+constexpr int ME_MINBLOCKS = 6;  // __launch_bounds__(128, N) of the motion-search kernel: registers/thread <= 65536 / (128 N)
 
 __device__ __forceinline__ int global_warp() { return (blockIdx.x * blockDim.x + threadIdx.x) >> 5; }
 __device__ __forceinline__ int total_warps() { return (gridDim.x * blockDim.x) >> 5; }
@@ -66,9 +68,7 @@ __global__ void fast_subpel_kernel(const S *a, int as, const S *b, int bs, int w
 // first), then draws the remaining searches, one warp each, from the caller's array in its own order.
 // class = ilog2(area), + 16 when the CTA-team form applies (speed 0, height a multiple of 8 rows per warp)
 constexpr int ME_TEAM_WARPS = WARPS_PER_CTA;
-#ifndef TB_ME_DRAW
-#define TB_ME_DRAW 4
-#endif
+constexpr int ME_DRAW = 4;
 __device__ __forceinline__ int me_class(int w, int h, int speed) {
   const int area = w * h, b = min(ilog2(max(area, 1)), 15);
   return (speed == 0 && area >= 2048 && (h % (8 * ME_TEAM_WARPS)) == 0) ? 16 + b : b;
@@ -81,7 +81,7 @@ struct MeClassOf {
   __device__ __forceinline__ int operator()(const tb_me_item_t &q) const {
     const int c = me_class(q.width, q.height, speed);
     if (c >= 16) return c;  // team items, largest first
-    if (quad && (int)q.width * (int)q.height <= 64 && (TB_ME_QUAD_SIZE16 || q.size != 16) && !((q.width | q.height) & 3) && !(q.ostride & 3) && !(q.rstride & 3) &&
+    if (quad && (int)q.width * (int)q.height <= 64 && !((q.width | q.height) & 3) && !(q.ostride & 3) && !(q.rstride & 3) &&
         !((uintptr_t)q.orig & 3))
       return 1;
     return -1;  // the others are drawn from the caller's array in its own order
@@ -127,12 +127,12 @@ template <class Item, class F> __global__ void sched_scatter_kernel(const Item *
 
 template <class S, int TW>
 __device__ __noinline__ void me_run_item(const tb_me_item_t *items, int it, const int16_t *cand, int bitdepth, int speed, int bip, int fw, int fh, tb_me_result_t *out,
-                                            unsigned long long *stats, MeTeam<TW> &tm, SubpelShared *sps) {
+                                            unsigned long long *stats, MeTeam<TW> &tm) {
   tb_me_item_t q = items[it];
   MeCtx c;
   c.size = q.size; c.width = q.width; c.height = q.height; c.sign = q.sign; c.s = q.sign ? -1 : 1;
   c.xpos = q.xpos; c.ypos = q.ypos; c.fw = fw; c.fh = fh; c.bitdepth = bitdepth; c.speed = speed; c.bip = bip;
-  c.mvpx = q.mvp_x; c.mvpy = q.mvp_y; c.lambda = q.lambda; c.n_int = 0; c.n_sub = 0; c.sps = sps;
+  c.mvpx = q.mvp_x; c.mvpy = q.mvp_y; c.lambda = q.lambda; c.n_int = 0; c.n_sub = 0;
   int mx, my;
   uint32_t cost;
   warp_motion_estimate<S, TW>((const S *)q.orig, q.ostride, (const S *)q.ref, q.rstride, c, q.mvc_x, q.mvc_y, cand + 2 * (size_t)q.cand_ofs, q.ncand, mx, my, cost, tm);
@@ -149,18 +149,12 @@ __device__ __noinline__ void me_run_item(const tb_me_item_t *items, int it, cons
 }
 
 template <class S>
-__global__ void __launch_bounds__(CTA_THREADS, TB_ME_MINBLOCKS) me_batch_kernel(const tb_me_item_t *items, int n, const int *idx, int *meta, const int16_t *cand, int bitdepth,
+__global__ void __launch_bounds__(CTA_THREADS, ME_MINBLOCKS) me_batch_kernel(const tb_me_item_t *items, int n, const int *idx, int *meta, const int16_t *cand, int bitdepth,
                                                                                  int speed, int bip, int fw, int fh, tb_me_result_t *out, unsigned long long *stats) {
   __shared__ uint32_t xch[2 * ME_TEAM_WARPS * 32];
   __shared__ int s_next;
-#if TB_SUBPEL_SHARED
-  __shared__ SubpelShared sps_all[WARPS_PER_CTA];
-  SubpelShared *sps = &sps_all[threadIdx.x >> 5];
-#else
-  SubpelShared *sps = nullptr;
-#endif
   const int nteam = meta[96], nlisted = meta[99];
-  const int quad = TB_ME_QUAD && sizeof(S) == 1 && speed == 0;
+  const int quad = sizeof(S) == 1 && speed == 0;
   // phase 1: the CTA as a team on the large blocks
   {
     MeTeam<ME_TEAM_WARPS> tm;
@@ -171,7 +165,7 @@ __global__ void __launch_bounds__(CTA_THREADS, TB_ME_MINBLOCKS) me_batch_kernel(
       const int k = s_next;
       __syncthreads();
       if (k >= nteam) break;
-      me_run_item<S, ME_TEAM_WARPS>(items, idx[k], cand, bitdepth, speed, bip, fw, fh, out, stats, tm, sps);
+      me_run_item<S, ME_TEAM_WARPS>(items, idx[k], cand, bitdepth, speed, bip, fw, fh, out, stats, tm);
     }
   }
   // phase 2: the searches that are neither team nor quad items, one warp each, drawn four at a time from the caller's array
@@ -182,16 +176,15 @@ __global__ void __launch_bounds__(CTA_THREADS, TB_ME_MINBLOCKS) me_batch_kernel(
     tm.xch = nullptr; tm.warp = 0; tm.phase = 0;
     for (;;) {
       int k = 0;
-      if (lane_id() == 0) k = atomicAdd(&meta[100], TB_ME_DRAW);
+      if (lane_id() == 0) k = atomicAdd(&meta[100], ME_DRAW);
       k = __shfl_sync(FULL, k, 0);
       if (k >= n) break;
-      for (int it = k; it < min(k + TB_ME_DRAW, n); it++) {
+      for (int it = k; it < min(k + ME_DRAW, n); it++) {
         if (nlisted && cls(items[it]) >= 0) continue;
-        me_run_item<S, 1>(items, it, cand, bitdepth, speed, bip, fw, fh, out, stats, tm, sps);
+        me_run_item<S, 1>(items, it, cand, bitdepth, speed, bip, fw, fh, out, stats, tm);
       }
     }
   }
-#if TB_ME_QUAD
   // phase 3: the listed small blocks (8-bit, <= 64 samples), four per warp (quad_motion_estimate).  They come last: the launch
   // ends on its cheapest searches, and the two code paths do not alternate in the instruction cache.
   if (sizeof(S) == 1) {
@@ -227,7 +220,6 @@ __global__ void __launch_bounds__(CTA_THREADS, TB_ME_MINBLOCKS) me_batch_kernel(
       __syncwarp();
     }
   }
-#endif
 }
 
 template <class S>
@@ -575,7 +567,7 @@ __device__ __noinline__ void tx_big_chain(const tb_txfm_item_t &q, int bitdepth,
 // (thread_txfm4 in registers, thread_txfm8 in per-thread local arrays; consecutive items are spatial neighbours, so the
 // lanes' loads and stores coalesce).
 template <class S>
-__global__ void __launch_bounds__(CTA_THREADS, TB_TX_MINBLOCKS) txfm_chain_kernel(const tb_txfm_item_t *items, int n, const int *idx, int *meta, int bitdepth, tb_txfm_result_t *out) {
+__global__ void __launch_bounds__(CTA_THREADS, TX_MINBLOCKS) txfm_chain_kernel(const tb_txfm_item_t *items, int n, const int *idx, int *meta, int bitdepth, tb_txfm_result_t *out) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ unsigned long long red[WARPS_PER_CTA];
   __shared__ int bc, s_next;

@@ -18,9 +18,7 @@
 #define TB_LDF(p) __ldcg(p)
 #define TB_ROLL _Pragma("unroll 1")  // loops stay loops: the kernel is bound by instruction fetch, not by loop overhead
 #define TB_ME_STAGE_PROF 1  // cycles per search stage (telescope, candidates, hexagon, half-pel, quarter-pel) of blocks <= 16 in the kernel's counters
-#ifndef TB_SAD_ROWS
 #define TB_SAD_ROWS 1  // integer-position SADs of blocks >= 32 bytes wide: lanes along the row (multi_sad_rows)
-#endif
 #define tb tb_rdo_tu
 #include <cstdio>
 #include <cstdlib>
@@ -477,7 +475,7 @@ template <class S> struct DevBackend {
     sync();
     MeCtx c;
     c.size = size; c.width = w; c.height = h; c.sign = sign; c.s = sign ? -1 : 1; c.xpos = xpos; c.ypos = ypos; c.fw = F->width; c.fh = F->height;
-    c.bitdepth = F->bitdepth; c.speed = F->speed; c.bip = F->enable_bipred; c.mvpx = mvp.x; c.mvpy = mvp.y; c.lambda = lambda; c.n_int = 0; c.n_sub = 0; c.sps = nullptr;
+    c.bitdepth = F->bitdepth; c.speed = F->speed; c.bip = F->enable_bipred; c.mvpx = mvp.x; c.mvpy = mvp.y; c.lambda = lambda; c.n_int = 0; c.n_sub = 0;
     for (int k = 0; k < 5; k++) c.cyc[k] = 0;
     MeTeam<1> tm;
     tm.xch = nullptr; tm.warp = 0; tm.phase = 0;
@@ -579,13 +577,8 @@ template <class S> struct DevBackend {
   }
 };
 
-#ifndef TB_RDO_WARPS
-#define TB_RDO_WARPS 8
-#endif
-#ifndef TB_RDO_CTAS_PER_SM
-#define TB_RDO_CTAS_PER_SM 1
-#endif
-constexpr int RDO_WARPS = TB_RDO_WARPS;  // warps per CTA: 8 x 32 threads x 255 registers = the whole register file of an SM
+constexpr int RDO_WARPS = 8;        // warps per CTA: 8 x 32 threads x 255 registers = the whole register file of an SM
+constexpr int RDO_CTAS_PER_SM = 1;  // two CTAs per SM (128 registers) measured slower than one (profiles/r2_ncu_rdo_summary.md)
 
 // One row of super blocks of one frame of the batch.  Rows are the unit a CTA claims; super blocks inside a row are sequential.
 struct RowDesc { int frame, row, nsbx, pad; };
@@ -599,7 +592,7 @@ enum { CTL_REMAINING = 0, CTL_ERROR = 1, CTL_EVENT = 2 /* bumped after every fin
 // so a CTA never holds an SM while it waits for a neighbour: a row migrates between CTAs at super-block boundaries (all per-super-block
 // state is re-initialised by process_sb; data of other super blocks is read through L2, see TB_LDF above).
 template <class S>
-__global__ void __launch_bounds__(32 * RDO_WARPS, TB_RDO_CTAS_PER_SM)
+__global__ void __launch_bounds__(32 * RDO_WARPS, RDO_CTAS_PER_SM)
     rdo_batch_kernel(const FrameCtx<S> *ctxs, const RowDesc *rows, int nrows, Work<S> *works, int *prog, int *claimed, int *ctl, unsigned long long *prof_out) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   RdoCta &cta = *(RdoCta *)smem_raw;
@@ -842,7 +835,6 @@ template <class S> int batch_launch(tb_rdo_batch *b, int n_active, cudaStream_t 
   if (!b->sms) { int dev = 0; CK(cudaGetDevice(&dev)); CK(cudaDeviceGetAttribute(&b->sms, cudaDevAttrMultiProcessorCount, dev)); }
   // persistent grid: every CTA is resident (a CTA may spin until a neighbour publishes), never more CTAs than rows
   int grid = b->sms * (per_sm[sizeof(S)] > 0 ? per_sm[sizeof(S)] : 1);
-  if (const char *e = getenv("TB_RDO_GRID")) { const int v = atoi(e); if (v > 0 && v < grid) grid = v; }
   if (grid > nrows) grid = nrows;
   if (grid > b->grid_cap) {
     cudaFree(b->works); b->works = nullptr; b->grid_cap = 0;

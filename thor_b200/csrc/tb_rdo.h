@@ -24,9 +24,6 @@
 #include <stdint.h>
 #include "../../include/thor_b200.h"
 
-#ifndef TBR_NO_OVERLAP
-#define TBR_NO_OVERLAP 0  // 1: every block through the serial form of mode_decision_rdo (A/B)
-#endif
 // TBR_NI: the functions of the control flow exist ONCE in the device code (no inlining at their many call sites): the RD loop is one kernel whose warps run
 // different parts of it at the same time, and an all-inlined build (2.5 MB of SASS) lives on instruction fetches from L2
 #ifdef __CUDACC__
@@ -1060,7 +1057,7 @@ template <class S, class B> struct Rdo {
   }
 
   TBR_HD uint32_t mode_decision_rdo(BlockInfo &bi, int *owner) {
-    if (F.frame_type != I_FRAME && F.speed == 0 && bi.bwidth == bi.size && bi.bheight == bi.size && bi.size <= MAX_TR && be.nwarps() > 1 && !TBR_NO_OVERLAP)
+    if (F.frame_type != I_FRAME && F.speed == 0 && bi.bwidth == bi.size && bi.bheight == bi.size && bi.size <= MAX_TR && be.nwarps() > 1)
       return mode_decision_overlap(bi, owner);
     return mode_decision_serial(bi, owner);
   }
